@@ -55,11 +55,31 @@ def parse():
     p.add_argument("--latency", action="store_true", help="accepted for compatibility: the batch-1 latency leg now always runs")
     p.add_argument("--no-latency", action="store_true",
                    help="skip the per-token decode latency leg at batch 1 (R=2 rows under CFG, AR sampling only, < 2 s)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="after the timed steps, write the fp32 pixels the last timed step returned (rank 0) as DIR/pixels.npy, so that "
+                        "two builds can be compared output for output; the inputs depend only on the arguments")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
 
 
 def log(msg):
     print(f"[bench {time.strftime('%H:%M:%S')}] {msg}", file=sys.stderr, flush=True)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, pixels):
+    """Write pixels [B, 3, H, W] as dirname/pixels.npy (float32). A batch over DUMP_BYTES keeps every k-th image (0, k, 2k, ...)
+    with the smallest k that fits."""
+    import numpy as np
+    arr = pixels.detach().float().cpu().numpy()
+    stride = -(-arr.nbytes // DUMP_BYTES)
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "pixels.npy"), np.ascontiguousarray(arr[::stride]))
+    log(f"wrote {dirname}/pixels.npy: images 0::{stride} of {arr.shape[0]}, shape {list(arr[::stride].shape)}")
 
 
 def host_cores():
@@ -397,11 +417,12 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """Run fn() `steps` times between CUDA events; returns the elapsed ms and what the last call returned."""
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
         ev0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         pipe.wait()            # every decode (and D2H) submitted above is inside the timed region
         ev1.record()
         barrier()
@@ -410,7 +431,7 @@ def run_ours(args):
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms
+        return ms, out
 
     labels_dev = cond_t2i if args.t2i else torch.randint(0, 1000, (B,), device=dev)
     log(f"rank {rank}: models ready, warming up")
@@ -427,9 +448,9 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     lib.lg_reset_launch_count()
-    ms = timed(lambda: step_resident(labels_dev), args.steps)
+    ms, last_pixels = timed(lambda: step_resident(labels_dev), args.steps)
     launches = int(lib.lg_launch_count())
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     clocks = sampler.stop() if rank == 0 else None
     log(f"rank {rank}: timed {ms / args.steps:.1f} ms/step resident, {ms_e2e / args.steps:.1f} ms/step e2e")
     value = world * B * args.steps / (ms / 1000.0)
@@ -645,6 +666,8 @@ def run_ours(args):
             line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": host_cores(), "kind": "port",
                                     "sample": f"failed: {type(ex).__name__}: {str(ex)[-300:]}"}
         log("cpu baseline leg done")
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_pixels)
     if rank == 0:
         emit(line)
     if world > 1:

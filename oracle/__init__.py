@@ -10,9 +10,9 @@ named in BASELINE.json:north_star:
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs may import this
 package, and only as the checker (or the timed CPU baseline) — never as a product path.
 
-Pinning: the reference is pure Python and imports in the authoring container, so the oracle is pinned
-against the LIVE reference (tests/test_oracle_vs_reference.py, skipped where /root/reference is absent)
-and against golden vectors the reference produced (tests/golden/*.pt, generator tests/golden/make_golden.py).
+Pinning: the oracle is pinned against outputs the reference itself produced on stored cases (tests/golden/*.pt and
+reference_surface.json, generator tests/golden/make_golden.py; checked by tests/test_oracle_vs_reference.py and
+tests/test_oracle_golden.py).
 """
 from .gpt_oracle import GPTOracle, rope_table_2d_oracle   # noqa: F401
 from .sampling_oracle import sample_oracle, top_k_top_p_oracle, cfg_mix_oracle   # noqa: F401

@@ -8,7 +8,7 @@ Restates, op for op and in the model dtype, the inference branches of
                                     LabelEmbedder :78-83, CaptionEmbedder/MLP :110-131
   autoregressive/models/generate.py prefill :77-86, decode_one_token :89-102, decode_n_tokens :105-123,
                                     generate :126-176
-over a plain state_dict (reference tensor names).  Pinned against the live reference by
+over a plain state_dict (reference tensor names).  Pinned against reference outputs by
 tests/test_oracle_vs_reference.py and against tests/golden/gpt_*.pt.
 """
 from __future__ import annotations

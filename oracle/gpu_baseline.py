@@ -1,7 +1,7 @@
 """GPU stand-in for "the reference's own PyTorch path on the same B200" (BASELINE.md §3.1) — BENCH INFRASTRUCTURE ONLY.
 
-/root/reference cannot travel to the GPU box, so the number north_star asks us to beat (reference PyTorch-GPU images/sec)
-is measured with the oracle, which is pinned bit-identically to the live reference (tests/test_oracle_vs_reference.py) and
+The reference sources are not part of this repository, so the number north_star asks us to beat (reference PyTorch-GPU
+images/sec) is measured with the oracle, which is pinned bit-identically to the reference (tests/test_oracle_vs_reference.py) and
 runs the same torch ops in the same order:
 
   * precision as the reference CLI sets it: bf16 GPT (`sample_c2i.py:38,46`), fp32 VQ with TF32 allowed

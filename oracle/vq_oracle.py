@@ -6,7 +6,7 @@ Restates tokenizer/tokenizer_image/vq_model.py over a plain state_dict:
   Normalize = GroupNorm(32, C, eps=1e-6) :359-362, nonlinearity (swish) :354-356,
   VectorQuantizer.forward index path :215-233,
   VQModel.encode :41-45 -> Encoder.forward :100-124 (Downsample :389-397) -> quant_conv -> VectorQuantizer.forward.
-Pinned against the live reference (tests/test_oracle_vs_reference.py) and tests/golden/vq_*.pt.
+Pinned against reference outputs (tests/test_oracle_vs_reference.py) and tests/golden/vq_*.pt.
 """
 from __future__ import annotations
 

@@ -7,7 +7,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-REFERENCE = "/root/reference"
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 
@@ -23,12 +22,3 @@ def pytest_collection_modifyitems(config, items):
     for item in items:
         if "gpu" in item.keywords:
             item.add_marker(skip)
-
-
-@pytest.fixture(scope="session")
-def reference_path():
-    if not os.path.isdir(os.path.join(REFERENCE, "autoregressive")):
-        pytest.skip("reference checkout not present (it never is on the GPU box)")
-    if REFERENCE not in sys.path:
-        sys.path.insert(0, REFERENCE)
-    return REFERENCE

@@ -1,7 +1,6 @@
 """CPU: CLI flag parity with the reference scripts, and the N>1 host logic (weight broadcast, sharding, seeds)
 over gloo with world_size 2."""
 import os
-import re
 import socket
 import sys
 
@@ -10,19 +9,18 @@ import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
-from conftest import ROOT
-
-
-def _ref_flags(path):
-    return set(re.findall(r'add_argument\(\s*"(--[a-z0-9\-]+)"', open(path).read()))
+from conftest import GOLDEN, ROOT
 
 
 @pytest.mark.parametrize("script", ["sample_c2i", "sample_t2i", "sample_c2i_ddp"])
-def test_cli_accepts_every_reference_flag(reference_path, script):
+def test_cli_accepts_every_reference_flag(script):
+    """Every flag the reference's sampling script defines (tests/golden/reference_surface.json, make_golden.py)."""
     import importlib
+    import json
     mod = importlib.import_module(f"llamagen_b200.sample.{script}")
     ours = {a for act in mod.build_parser()._actions for a in act.option_strings}
-    ref = _ref_flags(os.path.join(reference_path, "autoregressive", "sample", f"{script}.py"))
+    ref = set(json.load(open(os.path.join(GOLDEN, "reference_surface.json")))["cli_flags"][script])
+    assert ref
     assert ref <= ours, f"missing flags: {sorted(ref - ours)}"
 
 

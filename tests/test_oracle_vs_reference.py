@@ -1,105 +1,83 @@
-"""CPU, authoring container only: the oracle against the LIVE reference on fresh seeds (skipped on the GPU
-box, where /root/reference does not exist)."""
+"""CPU: the oracle (and the product's RoPE table, registries and center crop) against outputs of the reference
+itself, recorded by tests/golden/make_golden.py from the original LlamaGen sources into tests/golden/reference_cases.pt
+and tests/golden/reference_surface.json."""
+import json
+import os
+
 import pytest
 import torch
 
+from conftest import GOLDEN
 from oracle import GPTOracle, VQOracle, rope_table_2d_oracle
+from util import synth_state_dict, synth_tensor, tensor_digest
+
+CASES = torch.load(os.path.join(GOLDEN, "reference_cases.pt"), map_location="cpu", weights_only=False)
+SURFACE = json.load(open(os.path.join(GOLDEN, "reference_surface.json")))
+
+
+def _shapes(sd):
+    return {k: list(v.shape) for k, v in sd.items()}
 
 
 @pytest.mark.parametrize("model_type,cls", [("c2i", 1), ("t2i", 120)])
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
-def test_generate_matches_live_reference(reference_path, model_type, cls, dtype):
-    from autoregressive.models.generate import generate
-    from autoregressive.models.gpt import ModelArgs, Transformer
-    torch.manual_seed(11)
-    cfg = dict(n_layer=2, n_head=2, dim=128, vocab_size=256, block_size=16, cls_token_num=cls, model_type=model_type,
-               num_classes=7, caption_dim=64, norm_eps=1e-5, rope_base=10000)
-    m = Transformer(ModelArgs(**cfg)).eval()
-    m.output.weight.data.normal_(std=0.02)
-    m = m.to(dtype)
-    B = 2
+def test_generate_matches_live_reference(model_type, cls, dtype):
+    c = CASES["generate"][f"{model_type}_{str(dtype).split('.')[-1]}"]
+    assert c["cfg"]["cls_token_num"] == cls
+    sd = {k: v.to(dtype) for k, v in synth_state_dict(c["weights"]).items()}
     if model_type == "c2i":
-        cond, em = torch.tensor([3, 6]), None
+        cond = c["cond"]
     else:
-        em = torch.zeros(B, cls)
-        em[0, -5:] = 1
-        em[1, -77:] = 1
-        cond = (torch.randn(B, cls, 64) * em[:, :, None]).to(dtype)
-    ref = generate(m, cond, 16, emb_masks=em, cfg_scale=3.0, temperature=1.0, top_k=0, top_p=1.0, sample_logits=False)
-    toks, _ = GPTOracle(m.state_dict(), cfg).generate(cond, 16, emb_masks=em, cfg_scale=3.0, sample_logits=False)
-    assert torch.equal(ref, toks)
+        s = c["cond_spec"]
+        cond = (synth_tensor(s["seed"], "cond", s["shape"], 0.0, s["bound"]) * c["emb_masks"][:, :, None]).to(dtype)
+    toks, _ = GPTOracle(sd, c["cfg"]).generate(cond, c["S"], emb_masks=c["emb_masks"], cfg_scale=c["cfg_scale"],
+                                              sample_logits=False)
+    assert torch.equal(c["tokens"], toks)
 
 
-def test_rope_table_matches_live_reference(reference_path):
-    from autoregressive.models.gpt import precompute_freqs_cis_2d
+def test_rope_table_matches_live_reference():
     from llamagen_b200.gpt import rope_table_2d
-    for grid, hd, cls in ((16, 64, 1), (24, 100, 1), (32, 64, 120)):
-        ref = precompute_freqs_cis_2d(grid, hd, 10000, cls)
-        assert torch.equal(ref, rope_table_2d_oracle(grid, hd, 10000, cls))
-        assert torch.equal(ref, rope_table_2d(grid, hd, 10000, cls))
+    for grid, hd, cls, digest in CASES["rope"]:
+        assert tensor_digest(rope_table_2d_oracle(grid, hd, 10000, cls)) == digest
+        assert tensor_digest(rope_table_2d(grid, hd, 10000, cls)) == digest
 
 
-def test_registry_matches_live_reference(reference_path):
+def test_registry_matches_live_reference():
     """Same keys, same parameter names and shapes as the reference registries (drop-in boundary §8b)."""
-    from autoregressive.models.gpt import GPT_models as RefGPT
     from llamagen_b200 import GPT_models
-    assert set(RefGPT) == set(GPT_models)
+    assert SURFACE["gpt_models"] == sorted(GPT_models)
     for kw in (dict(model_type="c2i", cls_token_num=1, block_size=256), dict(model_type="t2i", cls_token_num=120, block_size=256)):
-        a = RefGPT["GPT-B"](**kw).state_dict()
-        b = GPT_models["GPT-B"](**kw).state_dict()
-        assert {k: tuple(v.shape) for k, v in a.items()} == {k: tuple(v.shape) for k, v in b.items()}
+        assert _shapes(GPT_models["GPT-B"](**kw).state_dict()) == SURFACE["gpt_b"][kw["model_type"]]
 
 
-def test_vq_registry_matches_live_reference(reference_path):
-    from tokenizer.tokenizer_image.vq_model import VQ_models as RefVQ
+def test_vq_registry_matches_live_reference():
     from llamagen_b200 import VQ_models
-    assert set(RefVQ) == set(VQ_models)
-    for name in RefVQ:
-        a = RefVQ[name](codebook_size=16384, codebook_embed_dim=8).state_dict()
-        b = VQ_models[name](codebook_size=16384, codebook_embed_dim=8).state_dict()
-        assert {k: tuple(v.shape) for k, v in a.items()} == {k: tuple(v.shape) for k, v in b.items()}
+    assert SURFACE["vq_models"] == sorted(VQ_models)
+    for name in SURFACE["vq_models"]:
+        assert _shapes(VQ_models[name](codebook_size=16384, codebook_embed_dim=8).state_dict()) == SURFACE["vq"][name]
 
 
-def test_vq_decode_matches_live_reference(reference_path):
-    import torch.nn as nn
-    from tokenizer.tokenizer_image.vq_model import Decoder, VectorQuantizer
-    torch.manual_seed(5)
-    dec = Decoder(z_channels=32, ch=32, ch_mult=(1, 2, 2)).eval()
-    quant = VectorQuantizer(128, 8, 0.25, 0.0, True, True).eval()
-    pqc = nn.Conv2d(8, 32, 1).eval()
-    sd = {"decoder." + k: v for k, v in dec.state_dict().items()}
-    sd.update({"quantize.embedding.weight": quant.embedding.weight.data, "post_quant_conv.weight": pqc.weight.data,
-               "post_quant_conv.bias": pqc.bias.data})
-    codes = torch.randint(0, 128, (1, 9))
-    with torch.no_grad():
-        ref = dec(pqc(quant.get_codebook_entry(codes, [1, 8, 3, 3], True)))
-    assert torch.equal(ref, VQOracle(sd, ch_mult=(1, 2, 2)).decode_code(codes, [1, 8, 3, 3]))
+def test_vq_decode_matches_live_reference():
+    c = CASES["vq_decode"]
+    pix = VQOracle(synth_state_dict(c["weights"]), ch_mult=tuple(c["ch_mult"])).decode_code(c["codes"], c["shape"])
+    assert torch.equal(c["pixels"], pix)
 
 
-def test_vq_encode_matches_live_reference(reference_path):
-    import torch.nn as nn
-    from tokenizer.tokenizer_image.vq_model import Encoder, VectorQuantizer
-    torch.manual_seed(6)
-    enc = Encoder(ch=32, ch_mult=(1, 2, 2), z_channels=32).eval()
-    quant = VectorQuantizer(128, 8, 0.25, 0.0, True, True).eval()
-    qc = nn.Conv2d(32, 8, 1).eval()
-    sd = {"encoder." + k: v for k, v in enc.state_dict().items()}
-    sd.update({"quantize.embedding.weight": quant.embedding.weight.data, "quant_conv.weight": qc.weight.data,
-               "quant_conv.bias": qc.bias.data})
-    x = torch.rand(1, 3, 24, 16) * 2 - 1
-    with torch.no_grad():
-        zq, _, info = quant(qc(enc(x)))
-    q, idx = VQOracle(sd, ch_mult=(1, 2, 2)).encode(x)
-    assert torch.equal(idx, info[2]) and torch.equal(q, zq)
+def test_vq_encode_matches_live_reference():
+    c = CASES["vq_encode"]
+    q, idx = VQOracle(synth_state_dict(c["weights"]), ch_mult=tuple(c["ch_mult"])).encode(c["x"])
+    assert torch.equal(idx, c["indices"]) and torch.equal(q, c["quant"])
 
 
-def test_center_crop_matches_live_reference(reference_path):
+def test_center_crop_matches_live_reference():
     import numpy as np
     from PIL import Image
-    from dataset.augmentation import center_crop_arr
     from llamagen_b200.sample.vq_demo import center_crop
     rng = np.random.default_rng(1)
+    cases = iter(CASES["center_crop"])
     for shape in [(300, 420), (1100, 900), (256, 256), (513, 2000)]:
         im = Image.fromarray(rng.integers(0, 255, (*shape, 3), dtype=np.uint8))
         for s in (256, 384):
-            assert (np.array(center_crop(im, s)) == np.array(center_crop_arr(im, s))).all()
+            ref_shape, ref_s, digest = next(cases)
+            assert (tuple(ref_shape), ref_s) == (shape, s)
+            assert tensor_digest(torch.from_numpy(np.array(center_crop(im, s)))) == digest
